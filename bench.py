@@ -29,6 +29,8 @@ mm_projector -> text/media splice -> Qwen2-7B prefill (S = 257 visual + 22 text 
                   26-layer tower + projector + 28-layer prefill once, then a bounded number of decode
                   tokens through all 28 layers (no extrapolation); thread count swept and stated
 
+`--dump-outputs DIR`    after the timed steps, rank 0 writes what the last timed request computed as DIR/<name>.npy
+                        (last_step_outputs): inputs are seeded, so two builds can be compared output for output.
 `--impl reference`      the same CPU port as its own arm (rank 0 only).
 `--impl reference_gpu`  informational: HF transformers (SigLIP + Qwen2, sdpa, bf16, eager) on the same
                         B200 for the same request — the library path the reference would run.
@@ -126,6 +128,24 @@ def make_request(cfg, seed=1):
     ids = torch.randint(0, 151643, (PROMPT_TEXT_TOKENS,), generator=g).tolist()
     ids.insert(14, cfg.image_token_id)  # "<system/user text> <image> <question>"
     return pixels, torch.tensor([ids], dtype=torch.long)
+
+
+def last_step_outputs(emb, hid, dec):
+    """Host copies of what one request_device() step computed (8 MB for NVILA-8B): the spliced prompt
+    embeddings [S, hidden], the prefill's final hidden states [S, hidden] (before the last RMSNorm) and
+    the NEW_TOKENS greedy ids (float64, exact).  Must run before the next request reuses these buffers
+    (the prefill output is a static CUDA-graph buffer)."""
+    return {"inputs_embeds": emb[0].float().cpu().numpy(),
+            "prefill_hidden": hid.float().cpu().numpy(),
+            "output_ids": dec.hist[:NEW_TOKENS].double().cpu().numpy()}
+
+
+def write_outputs(outputs, out_dir):
+    import numpy as np
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    for name, arr in outputs.items():
+        np.save(out / f"{name}.npy", arr)
 
 
 def llm_weight_bytes(lc):
@@ -473,6 +493,7 @@ def run_ours(args):
     ev = lambda: torch.cuda.Event(enable_timing=True)
 
     vision_ms = []
+    last = {}  # the latest request_device() results, for --dump-outputs
 
     def request_device():
         """inputs resident in HBM; returns (t_ttft_ms, t_decode_ms)."""
@@ -489,6 +510,7 @@ def run_ours(args):
         e2.record()
         torch.cuda.synchronize()
         vision_ms.append(e0.elapsed_time(ea))  # SigLIP tower + projector + splice
+        last.update(emb=emb, hid=hid, dec=dec)
         return e0.elapsed_time(e1), e1.elapsed_time(e2), emb.shape[1]
 
     def request_e2e(n_new):
@@ -527,6 +549,7 @@ def run_ours(args):
         barrier()
         t_wall = time.perf_counter() - t_wall0
         launches_timed = _lib.LAUNCHES - launches0
+        outputs = last_step_outputs(**last) if args.dump_outputs else None
         # e2e through the public API (host buffers)
         e2e_full, e2e_first = [], []
         for _ in range(args.steps):
@@ -685,6 +708,8 @@ def run_ours(args):
         "cpu_baseline": cpu,
         "wall_s_timed_region": round(t_wall, 3),
     }
+    if outputs is not None:
+        write_outputs(outputs, args.dump_outputs)
     print(json.dumps(line))
     dist.destroy_process_group()
 
@@ -962,7 +987,13 @@ def main():
     ap.add_argument("--sp-steps", type=int, default=10)
     ap.add_argument("--profile", action="store_true",
                     help="profiling aid (ncu): 1 warm-up, 8 new tokens, no extra blocks; NOT a valid bench number")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed request's embeddings, prefill hidden states and ids as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     if args.profile:
         global NEW_TOKENS
         NEW_TOKENS = 8
